@@ -59,7 +59,16 @@ def parse():
                          "through cv2 in the reference arm (the whole Tracker::track); precomputed: corner candidates prepared "
                          "beforehand, identical for both arms")
     ap.add_argument("--batch-streams", type=int, default=8, help="extra leg: independent streams run concurrently on one GPU (BASELINE configs[3])")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of the device-resident leg returned as DIR/<name>.npy "
+                         "(float64): pose, state_x, state_P, update_info; the inputs are seeded, so two builds can be compared output "
+                         "for output (rank 0 only)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    return args
 
 
 # ----------------------------------------------------------------------------------------- workload
@@ -214,6 +223,7 @@ def bind_to_gpu_numa_node(local_rank):
 
 # ----------------------------------------------------------------------------------------- B200 arm
 _LAST_DRIVE = {}
+_LAST_POSE = {}
 _RAW = {}
 
 
@@ -341,6 +351,7 @@ def drive(L, vio, wl, K, W, dev, inloop, dev_inputs, flush, prefetch=False):
             got_pose = True
         i += 1
     torch.cuda.synchronize()
+    _LAST_POSE["pose"] = None if pose is None else np.array(pose, np.float64)     # what the last timed step returned (--dump-outputs)
     step_ms = [a.elapsed_time(b) for a, b in zip(ev0, ev1)]
     # where a step's wall time goes on the host: inside the C call, enqueueing (image copy + graph launch) and blocked in its one
     # synchronisation; what is left of the wall time per step is the Python / ctypes layer around the call
@@ -350,6 +361,17 @@ def drive(L, vio, wl, K, W, dev, inloop, dev_inputs, flush, prefetch=False):
     if stage_diag:
         _LAST_DRIVE["stage_us"] = [round(float(v), 1) for v in np.median(np.array(stages), 0)]
     return step_ms, wall, L.rvio_b200_kernel_launches() - launches0, i, infos
+
+
+def dump_outputs(directory, vio, pose, info):
+    """--dump-outputs: what a caller of the device-resident path holds after the last timed step -- the pose it returned (NaN while
+    the filter initialises), the filter state x / P read back from the handle, and the step's update counters (n_feat, accepted,
+    stacked rows, rows kept, rank flags).  A few hundred kB at most (configs[4]: P is 204 x 204)."""
+    x, P = vio.state()
+    os.makedirs(directory, exist_ok=True)
+    out = {"pose": np.full(7, np.nan) if pose is None else pose, "state_x": x, "state_P": P, "update_info": np.array(info)}
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, np.float64))
 
 
 def run_b200(args, cfg, wl, rank, world, local_rank):
@@ -409,6 +431,8 @@ def run_b200(args, cfg, wl, rank, world, local_rank):
         dev_ms, dev_wall, launches, used, infos = drive(L, vio, wl, K, W, dev, inloop, True, flush)
         host_dev = dict(_LAST_DRIVE)
         barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, vio, _LAST_POSE["pose"], infos[-1])
     # ---- bare H2D copy of one frame from pinned memory (what `e2e.sync` adds in front of every step)
     pin = torch.from_numpy(frames[0]).pin_memory(); dst = torch.empty(pin.shape, dtype=pin.dtype, device=dev)
     h0, h1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -996,9 +1020,8 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        steps = min(K, 120)                                               # bounded sample of the same workload
-        wl = make_workload(cfg, int(T_STATIC * cfg.fps) + 4 + W + steps + 30, SEED + args.config, args.detector == "precomputed")
-        r = run_reference(cfg, wl, steps, W, ncores, args.detector == "inloop")
+        wl = make_workload(cfg, int(T_STATIC * cfg.fps) + 4 + W + K + 30, SEED + args.config, args.detector == "precomputed")
+        r = run_reference(cfg, wl, K, W, ncores, args.detector == "inloop")
         fps = r["steps"] / r["t"]
         out = {"metric": "vio_frames_per_sec", "value": fps, "unit": "frames/s", "n_gpus": args.gpus, "steps": r["steps"], "warmup": W,
                "ms_per_step": 1e3 * r["t"] / r["steps"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,

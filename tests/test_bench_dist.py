@@ -3,6 +3,8 @@ gloo backend at world_size 2."""
 import os
 import sys
 
+import numpy as np
+import pytest
 import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
@@ -80,6 +82,31 @@ def test_legs_deadline_prints_the_line_from_completed_legs(tmp_path):
     assert "legs_deadline" in line and line["sharded"] is None and line["roofline"] is None
     out1 = subprocess.run([sys.executable, str(script), "1"], capture_output=True, text=True, env=env, timeout=120)
     assert out1.returncode == 0 and out1.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_dump_outputs_repeat_from_run_to_run(tmp_path):
+    """--dump-outputs writes the last timed step's pose, filter state and update counters as float64; two runs with the same
+    arguments write the same arrays (seeded inputs), and --steps is the number of timed steps."""
+    import json
+    import subprocess
+    env = dict(os.environ, RVIO_BENCH_SETTLE_STEPS="0")
+    runs = []
+    for k in range(2):
+        d = tmp_path / f"run{k}"
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "7", "--warmup", "3", "--no-extra-legs",
+                              "--no-cpu-baseline", "--batch-streams", "0", "--dump-outputs", str(d)],
+                             capture_output=True, text=True, env=env, timeout=600)
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads(out.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 7 and len(line["update_frames"]["rows_kept_flags"]) == 7
+        runs.append({n: np.load(d / f"{n}.npy") for n in ("pose", "state_x", "state_P", "update_info")})
+    a, b = runs
+    for n in a:
+        assert a[n].dtype == np.float64 and np.array_equal(a[n], b[n]), n
+    n_clones = (len(a["state_x"]) - 26) // 7
+    assert a["pose"].shape == (7,) and np.isfinite(a["pose"]).all()
+    assert a["state_P"].shape == (24 + 6 * n_clones,) * 2 and a["update_info"].shape == (5,)
 
 
 def test_no_undefined_names_in_the_python_sources():

@@ -11,10 +11,9 @@ import rvio_b200  # noqa: F401
 from rvio_b200 import synth
 from oracle import oracle as orc
 
-cv2 = pytest.importorskip("cv2")
-
 
 def _images():
+    cv2 = pytest.importorskip("cv2")        # the golden-fixture test below needs no cv2
     cfg = synth.baseline_config(1)
     st = synth.Stream(cfg, 4, 20260928, t_static=0.1)
     clahe = cv2.createCLAHE(3.0, (5, 5))
@@ -30,6 +29,7 @@ def _images():
 
 
 def test_min_eig_map_matches_cv2():
+    cv2 = pytest.importorskip("cv2")
     for cfg, img in _images():
         want = cv2.cornerMinEigenVal(img, 3, ksize=3)
         got = orc.min_eig_map(img)
